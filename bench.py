@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ICAFusion hot path on B200: 640x512 RGB+IR pairs/s end to end (+ roofline of the dominant kernel).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`):
     yolov5l_b16  (default)  configs[2]: yolov5l_ICAFusion, 640x512 synthetic RGB+IR, batch 16 per GPU, inference -- the largest
@@ -46,6 +46,23 @@ WORKLOADS = {
     "yolov5l_b16": dict(size="l", batch=16, H=512, W=640, desc="yolov5l_ICAFusion 640x512 synthetic RGB+IR, batch 16, inference"),
 }
 METRIC = "640x512 RGB+IR pairs/sec end-to-end"
+DUMP_LIMIT = 64 << 20       # bytes written by --dump-outputs
+
+
+def _to_host(arrays):
+    """name -> tensor  =>  name -> float32 numpy copy (taken now: graph outputs are overwritten by the next replay)."""
+    return {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+
+
+def _dump(outdir, host):
+    """--dump-outputs: DIR/<name>.npy per array."""
+    import numpy as np
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(outdir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(outdir, k + ".npy"), a)
 
 
 def _peaks():
@@ -161,8 +178,8 @@ def run_reference(args, wl):
     if rank != 0:
         return
     steps = max(1, args.steps)
-    # one "step" of this arm = one pair of the workload (a bounded sample of its batch); W warm-up pairs, K timed pairs, capped at 90 s
-    cb = cpu_reference_throughput(wl, budget_s=90.0, max_pairs=steps, warm=max(1, min(args.warmup, 3)))
+    # one "step" of this arm = one pair of the workload (a bounded sample of its batch); W warm-up pairs, K timed pairs
+    cb = cpu_reference_throughput(wl, budget_s=float("inf"), max_pairs=steps, warm=max(1, min(args.warmup, 3)))
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": "pairs/s", "n_gpus": args.gpus, "steps": steps,
             "warmup": args.warmup, "ms_per_step": round(1000.0 / cb["value"], 3), "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -214,6 +231,8 @@ def _measure(args, wl, K, Wm, dev, world, rank, local, primary=True):
     barrier()
     t_wall = time.perf_counter() - t_wall
     dev_ms = sum(s.elapsed_time(e) for s, e in ev)
+    if primary and args.dump_outputs and rank == 0:       # what the last timed replay returned: (z, logits, [x0, x1, x2])
+        _dump(args.dump_outputs, _to_host({"z": eng.z, "logits": eng.logits, **{f"x{i}": x for i, x in enumerate(eng.xs)}}))
     # ---------------- end-to-end timing through the public streaming call with host frames ----------------------
     # PipelinedDetector.infer_stream: per frame H2D (pinned uint8) -> forward -> D2H of the decoded predictions; the copy
     # of frame i+1 overlaps the forward of frame i (depth-2), the host blocks on the oldest frame in flight.
@@ -412,14 +431,26 @@ def _measure_train(args, wl, K, Wm, dev, world, rank, local):
         torch.cuda.synchronize()
 
     def timed(fn, n):
+        """(ms of n calls, what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(n):
-            fn()
+            out = fn()
         e1.record()
         barrier()
-        return e0.elapsed_time(e1)
+        return e0.elapsed_time(e1), out
+
+    dump = args.mode == "train" and args.dump_outputs and rank == 0
+    if dump:
+        n_all = sum(p.numel() for p in model.parameters())
+        pick = torch.randint(n_all, (1 << 20,), generator=torch.Generator().manual_seed(0)).to(dev)
+
+    def outputs(step_out):
+        """The step's (loss, loss_items) and a fixed sample of the parameters it updated, on the host."""
+        loss, items = step_out
+        params = torch.cat([p.detach().reshape(-1).float() for p in model.parameters()])
+        return _to_host({"loss": loss.reshape(1), "loss_items": items, "params_sample": params[pick]})
 
     def resident():
         return ts(rgb_d, ir_d, tg_d)
@@ -431,8 +462,9 @@ def _measure_train(args, wl, K, Wm, dev, world, rank, local):
     for _ in range(Wm):
         resident()
     n0 = ops.launch_count()
-    eager_ms = timed(resident, K)
+    eager_ms, last = timed(resident, K)
     launches = ops.launch_count() - n0
+    dumped = outputs(last) if dump else None
     # per-kernel split of one step (event pass on one stream)
     summ = {}
     if rank == 0:
@@ -469,11 +501,14 @@ def _measure_train(args, wl, K, Wm, dev, world, rank, local):
             return float(loss)
         for _ in range(2):
             resident()
-        res_ms = timed(resident, K)
+        res_ms, last = timed(resident, K)
+        dumped = outputs(last) if dump else None
     else:
         res_ms = eager_ms
+    if dump:
+        _dump(args.dump_outputs, dumped)
     e2e()
-    e2e_ms = timed(e2e, K)
+    e2e_ms, _ = timed(e2e, K)
     if gts is not None:
         gts.close()
     in_sync = None
@@ -488,7 +523,7 @@ def _measure_train(args, wl, K, Wm, dev, world, rank, local):
             with ts.model.no_sync():
                 return ts(rgb_d, ir_d, tg_d)
         local_only()
-        nosync_ms = timed(local_only, K)
+        nosync_ms, _ = timed(local_only, K)
     t = torch.tensor([res_ms, e2e_ms, nosync_ms, eager_ms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -644,7 +679,12 @@ def main():
     ap.add_argument("--train-steps", type=int, default=10)
     ap.add_argument("--mode", default="infer", choices=["infer", "train"], help="train: the JSON line's top-level metric is the training "
                     "step (BASELINE configs[3]; under torchrun it is the DDP step with its gradient all-reduce) instead of inference")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="after the timed steps, write what the timed path computed in "
+                    "its last step as DIR/<name>.npy (float32; rank 0): infer -> z, logits, x0..x2 of the detector; train -> loss, "
+                    "loss_items and a fixed sample of 2^20 parameter values after the step")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, wl)

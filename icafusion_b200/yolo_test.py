@@ -322,6 +322,8 @@ class Model(nn.Module):
         layers = list(self.model)
         y: List = [None] * len(layers)
         dev = rgb.device
+        if not ops.on_device(rgb):
+            raise RuntimeError("icafusion_b200 runs on CUDA tensors only (no CPU fallback)")
         dry = ops.dry_running()                   # shape-only walk on meta tensors (no streams, nothing launched)
         main = None if dry else torch.cuda.current_stream(dev)
         forked = {}                               # layer index -> side stream its result is being produced on

@@ -30,6 +30,9 @@ OUT = os.path.join(ROOT, "tests", "golden")
 HYP = dict(box=0.05, obj=1.0, cls=0.5, cls_pw=1.0, obj_pw=1.0, anchor_t=4.0, fl_gamma=0.0)
 CASE = dict(name="train_yolov5s_320", size="s", B=2, H=320, W=320, nt=12, seed=1234)
 BN_PROBES = ["model.0.bn", "model.4.cv3.bn", "model.10.bn", "model.22.conv1x1_out.bn"]
+# intra-op threads of the stored run.  The step's gradients move by up to ~1.5e-3 of their norm with the CPU summation order
+# (BatchNorm batch statistics in the backward), so whoever replays the step on the CPU uses the same thread count.
+THREADS = 8
 
 
 def synth_targets(nt: int, B: int, seed: int) -> np.ndarray:
@@ -50,6 +53,7 @@ def fingerprint(a: np.ndarray, key: str) -> np.ndarray:
 
 def main():
     warnings.filterwarnings("ignore")
+    torch.set_num_threads(THREADS)
     _, yolo = load_reference()
     from utils.loss import ComputeLoss
     c = CASE

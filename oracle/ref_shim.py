@@ -3,11 +3,11 @@
 The reference is pure Python/PyTorch but imports a few packages this image lacks
 (matplotlib, seaborn, thop, timm, pycocotools).  `load_reference()` installs inert
 stand-ins for those in `sys.modules`, puts the reference tree on `sys.path` and returns
-its `models.common` / `models.yolo_test` modules.  Nothing under /root/reference is
+its `models.common` / `models.yolo_test` modules.  Nothing in the reference tree is
 modified or copied.
 
-Only `oracle/gen_golden.py` and the `not gpu` tests that pin the oracle call this, and
-only inside the build container: the GPU box has no /root/reference.
+Only the `oracle/gen_golden*.py` generators call this; the tests replay what they stored
+under tests/golden/ and need no reference tree.
 """
 import importlib
 import os

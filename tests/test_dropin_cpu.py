@@ -1,42 +1,26 @@
-"""Drop-in proof for INTEGRATION.md section 2 (CPU only, needs the reference tree): a full-object checkpoint written by
-the REAL reference (``torch.save({'model': model})``, train.py:424-435) is unpickled into the shadow modules
-(``sys.modules['models.common'] = icafusion_b200.common`` etc.), goes through what ``attempt_load`` does
-(models/experimental.py:113-121: ``ckpt['model'].float().fuse().eval()``), loads the reference's state_dict with
-``strict=True`` and walks the product path (dry run: meta tensors, every kernel launch planned, none issued)."""
-import os
+"""Drop-in proof for INTEGRATION.md section 2 (CPU only): a full-object checkpoint written by the REAL reference
+(``torch.save({'model': model})``, train.py:424-435; stored in tests/golden/dropin_reference.npz by
+oracle/gen_golden_dropin.py) is unpickled into the shadow modules (``sys.modules['models.common'] = icafusion_b200.common``
+etc.), goes through what ``attempt_load`` does (models/experimental.py:113-121: ``ckpt['model'].float().fuse().eval()``),
+loads the reference's state_dict with ``strict=True`` and walks the product path (dry run: meta tensors, every kernel launch
+planned, none issued)."""
 import subprocess
 import sys
 import textwrap
 
-import pytest
 import torch
 
-from conftest import ROOT
-from oracle.ref_shim import REF_ROOT, reference_available
-
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference tree only exists in the build container")
+from conftest import ROOT, load_golden
+from oracle.gen_golden_dropin import COMMON_CLASSES, fill_state_dict, init_signature
 
 
 def _write_reference_checkpoint(path, sd_path):
-    """Runs in a child process so the reference's `models` package never shares sys.modules with the shadow modules."""
-    code = textwrap.dedent(f"""
-        import sys, torch, os
-        sys.path.insert(0, {ROOT!r})
-        from oracle import synth
-        from oracle.ref_shim import load_reference, REF_ROOT
-        common, yolo = load_reference()
-        cfg = os.path.join(REF_ROOT, "models", "transformer", "yolov5s_Transfusion_kaist.yaml")
-        model = yolo.Model(cfg, ch=3, nc=1)
-        shapes = {{k: tuple(v.shape) for k, v in model.state_dict().items()}}
-        model.load_state_dict(synth.synth_state_dict(shapes, 77), strict=False)
-        model.half()                                   # train.py:427 saves the half() model object
-        torch.save({{"epoch": 3, "model": model, "optimizer": None}}, {path!r})
-        torch.save(model.float().state_dict(), {sd_path!r})
-        print(type(model).__module__, len(shapes))
-    """)
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stderr[-2000:]
-    assert out.stdout.split()[0] == "models.yolo_test"
+    """The reference's checkpoint bytes and its state_dict (rebuilt from the stored layout, exactly what it held)."""
+    m, d = load_golden("dropin_reference")
+    with open(path, "wb") as f:
+        f.write(d["ckpt"].tobytes())
+    fill = fill_state_dict(m["sd"])
+    torch.save({k: fill[k] if k in fill else torch.from_numpy(d["sd:" + k]) for k, _, _ in m["sd"]}, sd_path)
 
 
 def test_reference_checkpoint_unpickles_into_shadow_modules(tmp_path):
@@ -88,24 +72,14 @@ def test_reference_checkpoint_unpickles_into_shadow_modules(tmp_path):
 def test_shadow_modules_export_the_reference_names():
     """Every class the Transfusion YAMLs / pickles name exists in the shadow modules with the reference's constructor
     signature (parameter names and defaults)."""
-    import inspect
     import icafusion_b200.common as C
     import icafusion_b200.yolo_test as Y
-    from oracle.ref_shim import load_reference
-    src_common = open(os.path.join(REF_ROOT, "models", "common.py")).read()
+    ref = load_golden("dropin_reference")[0]["signatures"]
+    for name in COMMON_CLASSES:
+        assert name in ref and hasattr(C, name), name
     for name in ("Conv", "Bottleneck", "C3", "SPPF", "Concat", "TransformerFusionBlock", "CrossTransformerBlock", "CrossAttention",
-                 "LearnableCoefficient", "LearnableWeights", "AdaptivePool2d"):
-        assert f"class {name}(" in src_common and hasattr(C, name), name
-    rc, ry = load_reference()
-    try:
-        for name in ("Conv", "Bottleneck", "C3", "SPPF", "Concat", "TransformerFusionBlock", "CrossTransformerBlock", "CrossAttention",
-                     "AdaptivePool2d"):
-            a, b = inspect.signature(getattr(rc, name).__init__), inspect.signature(getattr(C, name).__init__)
-            assert [(p.name, p.default) for p in a.parameters.values()] == [(p.name, p.default) for p in b.parameters.values()], name
-        for name in ("Model", "Detect"):
-            assert hasattr(Y, name)
-        a, b = inspect.signature(ry.Detect.__init__), inspect.signature(Y.Detect.__init__)
-        assert [p.name for p in a.parameters.values()] == [p.name for p in b.parameters.values()]
-    finally:
-        for k in [k for k in sys.modules if k == "models" or k.startswith("models.") or k == "utils" or k.startswith("utils.")]:
-            del sys.modules[k]      # keep the reference's packages out of the other tests' namespace
+                 "AdaptivePool2d"):
+        assert init_signature(getattr(C, name)) == ref[name], name
+    for name in ("Model", "Detect"):
+        assert hasattr(Y, name)
+    assert [p for p, _ in init_signature(Y.Detect)] == [p for p, _ in ref["Detect"]]

@@ -1,17 +1,15 @@
 """Host-side logic that needs no GPU: config generation, graph building, state_dict parity with the reference,
 filter packing layout, BN folding, pooling geometry."""
-import os
-
 import pytest
 import torch
 
+from conftest import load_golden
 from icafusion_b200 import Model, TransformerFusionBlock, ops
 from icafusion_b200.cfg import load_cfg, transfusion_kaist_cfg
 from icafusion_b200.common import AdaptivePool2d, Conv
 from icafusion_b200.yolo_test import fuse_conv_and_bn
 from oracle import icaf_oracle as O
 from oracle import synth
-from oracle.ref_shim import REF_ROOT, reference_available
 
 
 @pytest.mark.parametrize("size", ["s", "l"])
@@ -31,12 +29,10 @@ def test_state_dict_layout_matches_reference(size):
     assert abs(n_params / 1e6 - (23.26 if size == "s" else 120.25)) < 0.01     # SURVEY.md section 8(a)
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree only exists in the build container")
 @pytest.mark.parametrize("size", ["s", "l"])
 def test_generated_cfg_equals_reference_yaml(size):
-    import yaml
-    with open(os.path.join(REF_ROOT, "models", "transformer", f"yolov5{size}_Transfusion_kaist.yaml")) as f:
-        ref = yaml.safe_load(f)
+    """models/transformer/yolov5{s,l}_Transfusion_kaist.yaml as the reference parses it (stored by oracle/gen_golden_dropin.py)."""
+    ref = load_golden("dropin_reference")[0]["cfg"][size]
     mine = transfusion_kaist_cfg(size)
     for k in ("nc", "depth_multiple", "width_multiple", "anchors", "backbone", "head"):
         assert mine[k] == ref[k], k

@@ -108,14 +108,19 @@ def test_training_step_oracle_matches_reference_golden():
     """oracle.train_step (train-mode forward with BatchNorm batch statistics and the nearest DMFF tail, loss, autograd backward)
     reproduces the REAL reference's training step (tests/golden/train_yolov5s_320.npz, oracle/gen_golden_train.py): loss, a
     fingerprint of every parameter gradient, the set of parameters that receive no gradient, updated BN running statistics."""
-    from oracle.gen_golden_train import fingerprint, synth_targets
+    from oracle.gen_golden_train import THREADS, fingerprint, synth_targets
     m, d = load_golden("train_yolov5s_320")
     cfg = load_cfg(f"yolov5{m['size']}_Transfusion_kaist")
     sd = synth.synth_state_dict(synth.model_param_shapes(cfg), m["seed"])
     rgb, ir = synth.synth_images(m["B"], m["H"], m["W"], m["seed"])
     t = synth_targets(m["nt"], m["B"], m["seed"])
     assert np.array_equal(t, d["targets"])
-    loss, items, grads, pred, state = O.train_step(sd, cfg, rgb, ir, torch.from_numpy(t), m["hyp"], m["gr"])
+    n_threads = torch.get_num_threads()
+    torch.set_num_threads(THREADS)                                  # the stored run's summation order
+    try:
+        loss, items, grads, pred, state = O.train_step(sd, cfg, rgb, ir, torch.from_numpy(t), m["hyp"], m["gr"])
+    finally:
+        torch.set_num_threads(n_threads)
     got = np.concatenate([loss.numpy().reshape(1), items.numpy()])
     assert np.allclose(got, d["out"], rtol=1e-4, atol=1e-6), (got, d["out"])
     assert sorted(grads) == sorted(m["params"])                     # the same 30 parameters stay without a gradient
